@@ -1,6 +1,6 @@
 """bench.py -- agent-env-steps/sec of the CACC + A2C + NeurComm hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one full update of the hot path over one batch: n_step (60) env steps of B parallel
@@ -20,6 +20,10 @@ backward cell kernel and the weight-gradient GEMM.  `cpu_baseline` times the res
 unavailable) on the host cores.  `configs` holds the other BASELINE.json configurations at their TOTAL env
 counts split over the N ranks (cfg2 strong-scaling point, cfg3 CommNet, cfg4 DIAL, cfg5 5x5 grid), and
 `dropin_b1` the reference-facing list/NumPy API at one env (main.py train's loop).
+
+`--dump-outputs DIR` writes what the last of the K timed updates computed (rank 0) as DIR/<name>.npy, so that two
+builds run with the same arguments can be compared output for output: the inputs (configs, seeds, Philox streams)
+are identical from run to run.
 """
 import argparse
 import json
@@ -39,15 +43,21 @@ N_ENV = 4096
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=20)
+    ap.add_argument('--steps', type=int, default=20, help='timed updates of the headline workload (and of its e2e arm)')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed update as DIR/<name>.npy')
     ap.add_argument('--n-env', type=int, default=N_ENV, help='parallel envs per GPU')
     ap.add_argument('--config', default=CONFIG)
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--no-extra', action='store_true', help='skip the `configs` block and the B=1 drop-in timing')
-    return ap.parse_args()
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs needs --impl ours')
+    return args
 
 
 def load_cfg(name, **env_over):
@@ -209,6 +219,37 @@ def build(config, B, rank, **env_over):
     return cp, env, model
 
 
+DUMP_BYTES = 63 * 10 ** 6       # array data of --dump-outputs; with the .npy headers the directory stays under 64 MB
+
+
+def dump_outputs(e, out_dir):
+    """Writes what the last update handed its caller as <out_dir>/<name>.npy (float32 or float64): the updated weights,
+    the gradient and its norm, the per-agent loss terms, and per env the rollout (global rewards, dones, actions, pi,
+    values, observations after each step, bootstrap values) with its n-step returns and advantages.  When all envs
+    do not fit in DUMP_BYTES, a fixed seeded subset of them is written; env_index.npy lists which."""
+    import numpy as np
+    import torch
+    T, B = e.T_cur, e.B
+    whole = {'params': e.params, 'grads': e.grads, 'grad_norm': e.norm_out}
+    # (tensor, env axis); slot t + 1 of obs / fp / done holds what step t produced
+    per_env = {'rewards': (e.grew_buf[:T], 1), 'dones': (e.done_buf[1:T + 1], 1), 'actions': (e.act_buf[:T].float(), 2),
+               'pi': (e.fp_buf[1:T + 1], 2), 'values': (e.val_buf[:T], 2), 'obs': (e.obs_buf[1:T + 1], 2),
+               'bootstrap_values': (e.R_end, 1), 'returns': (e.Rs[:T], 2), 'advantages': (e.Advs[:T], 2)}
+    fixed = sum(t.numel() * t.element_size() for t in whole.values())
+    env_bytes = sum(t.numel() // B * t.element_size() for t, _ in per_env.values()) + 8
+    k = min(B, (DUMP_BYTES - fixed) // env_bytes)
+    idx = np.sort(np.random.RandomState(0).choice(B, k, replace=False))
+    out = {n: t.cpu().numpy() for n, t in whole.items()}
+    out.update(e.losses())
+    sel = torch.as_tensor(idx, device=e.device)
+    out.update({n: t.index_select(d, sel).cpu().numpy() for n, (t, d) in per_env.items()})
+    out['env_index'] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for n, a in out.items():
+        assert a.dtype in (np.float32, np.float64), (n, a.dtype)
+        np.save(os.path.join(out_dir, n + '.npy'), a)
+
+
 class Runner:
     """Device-timed and end-to-end throughput of whole updates for one configuration."""
 
@@ -238,7 +279,7 @@ class Runner:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return float(ms.item())
 
-    def measure(self, env, model, steps, warmup, e2e=True, clocks=False):
+    def measure(self, env, model, steps, warmup, e2e=True, clocks=False, dump=None):
         import torch
         from deeprl_network_b200.utils import VecTrainer
         e = model.engine
@@ -263,6 +304,8 @@ class Runner:
         ms = self.timed(vt.update, steps)
         if sampler is not None:
             out['clocks'] = sampler.summary()
+        if dump is not None:
+            dump_outputs(e, dump)          # before the e2e arm below trains the same model further
         out['value'] = steps * per_update * self.world / (ms * 1e-3)
         out['ms_per_step'] = ms / steps
         if e2e:
@@ -457,7 +500,8 @@ def main():
     cp, env, model = build(args.config, B, rank)
     e = model.engine
     T, N = e.T, e.N
-    head = runner.measure(env, model, args.steps, args.warmup, e2e=not args.no_e2e, clocks=True)
+    head = runner.measure(env, model, args.steps, args.warmup, e2e=not args.no_e2e, clocks=True,
+                          dump=args.dump_outputs if rank == 0 else None)
     peaks = {}
     try:
         peaks = json.load(open(os.path.join(ROOT, 'MEASURED_PEAKS.json')))

@@ -12,7 +12,9 @@ Reference pieces executed here:
      as a default argument at import time -- SURVEY 8c)
 """
 import configparser
+import glob
 import hashlib
+import json
 import os
 import sys
 import types
@@ -414,6 +416,17 @@ def hetero_case(agent):
     return out
 
 
+def configs_case():
+    """Every CACC .ini of the reference as parsed key/value pairs, by file and section (what config/ must reproduce)."""
+    out = {}
+    for path in sorted(glob.glob(os.path.join(REF, 'config', 'config_*_catchup.ini')) +
+                       glob.glob(os.path.join(REF, 'config', 'config_*_slowdown.ini'))):
+        cp = configparser.ConfigParser()
+        cp.read(path)
+        out[os.path.basename(path)] = {s: dict(cp[s]) for s in cp.sections()}
+    return out
+
+
 def scheduler_case(au):
     s1 = au.Scheduler(5e-4, decay='constant')
     s2 = au.Scheduler(5e-4, 1e-4, 1e6, decay='linear')
@@ -488,6 +501,11 @@ def main():
         out = hetero_case(agent)
         np.savez_compressed(os.path.join(HERE, name + '.npz'), **out)
         print(name, 'trace', out['trace'].shape, 'n_var', len(out['names']))
+    path = os.path.join(HERE, 'reference_configs.json')
+    if not os.path.exists(path) or '--force' in sys.argv:
+        with open(path, 'w') as f:
+            json.dump(configs_case(), f, indent=1, sort_keys=True)
+        print('reference_configs.json')
     if '--force' not in sys.argv:
         return
     for name, alpha, multi in [('buffer_ma_global', -1, True), ('buffer_ma_spatial09', 0.9, True),
