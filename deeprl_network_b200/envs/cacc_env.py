@@ -40,9 +40,50 @@ def grid_masks(side):
     return (dist == 1).astype(int), dist
 
 
+def seed_uniforms(seeds, n_platoon):
+    """float64 [P, B]: column k holds the uniforms ``CACCEnv.reset(test_ind=k)`` draws for test seed ``seeds[k]``
+    (``np.random.seed(seed)``, then one ``rand()`` per platoon in order).  A private RandomState gives the same
+    values as the legacy global seeding and leaves the global NumPy stream untouched."""
+    out = np.empty((int(n_platoon), len(seeds)), dtype=np.float64)
+    for k, s in enumerate(seeds):
+        out[:, k] = np.random.RandomState(int(s)).rand(int(n_platoon))
+    return out
+
+
+def control_row(episode, t, dt, action, global_reward):
+    """One row of ``{scenario}_{agent}_control.csv`` (envs/cacc_env.py:81-137): step t of an episode."""
+    return {'episode': episode, 'time_sec': t * dt, 'step': t,
+            'action': ','.join(['%d' % a for a in action]), 'reward': global_reward}
+
+
+def traffic_frame(episode, dt, rewards, trace, n_agent):
+    """The ``_traffic.csv`` block of one episode.  rewards: [0] + the per-step global rewards; trace float64
+    [steps + 1, 3, N] = (h, v, u) of every vehicle, the reset state first."""
+    import pandas as pd
+    tr = np.asarray(trace)
+    hs, vs, us = tr[:, 0], tr[:, 1], tr[:, 2]
+    df = pd.DataFrame()
+    df['episode'] = np.ones(len(hs)) * episode
+    df['time_sec'] = np.arange(len(hs)) * dt
+    df['reward'] = np.array(rewards)
+    df['lead_headway_m'] = hs[:, 0]
+    df['avg_headway_m'] = np.mean(hs[:, 1:], axis=1)
+    df['std_headway_m'] = np.std(hs[:, 1:], axis=1)
+    df['avg_speed_mps'] = np.mean(vs, axis=1)
+    df['std_speed_mps'] = np.std(vs, axis=1)
+    df['avg_accel_mps2'] = np.mean(us, axis=1)
+    df['std_accel_mps2'] = np.std(us, axis=1)
+    for i in range(n_agent):
+        df['headway_%d_m' % (i + 1)] = hs[:, i]
+        df['velocity_%d_mps' % (i + 1)] = vs[:, i]
+        df['accel_%d_mps2' % (i + 1)] = us[:, i]
+    return df
+
+
 class CACCEnv:
     def __init__(self, config, n_env=None, device=None):
         L.require_cuda()
+        self.config = config
         self._load_config(config)
         if n_env is not None:
             self.n_env = int(n_env)
@@ -154,6 +195,18 @@ class CACCEnv:
                                         L.ptr(self.collision_dev), L.ptr(self.v_init), L.ptr(obs), obs.shape[-1],
                                         L.ptr(rew), L.ptr(grew), L.ptr(done), L.stream()), 'nmarl_cacc_step')
 
+    def reset_seeds(self, seeds, obs_out=None, fp_out=None):
+        """Test-mode reset of all B envs in one launch: env k starts the episode ``reset(test_ind)`` would start for
+        test seed ``seeds[k]`` (same uniforms, see ``seed_uniforms``).  Sets ``train_mode = False``."""
+        seeds = [int(s) for s in seeds]
+        if len(seeds) != self.n_env:
+            raise ValueError('reset_seeds: %d seeds for %d envs' % (len(seeds), self.n_env))
+        self._u01.copy_(torch.from_numpy(seed_uniforms(seeds, self._u01.shape[0])))
+        self.train_mode = False
+        self.reset_device(u01=self._u01, obs_out=obs_out, fp_out=fp_out)
+        self.collision = False
+        self.t = 0
+
     @property
     def cfg_seed(self):
         return getattr(self, '_cfg_seed', 0)
@@ -251,29 +304,19 @@ class CACCEnv:
         self._trace.append(torch.stack([self.hs[:, 0], self.vs[:, 0], self.us[:, 0]]).cpu().numpy())
 
     def _log_control_data(self, action, global_reward):
-        self.control_data.append({'episode': self.cur_episode, 'time_sec': self.t * self.dt, 'step': self.t,
-                                  'action': ','.join(['%d' % a for a in action]), 'reward': global_reward})
+        self.control_data.append(control_row(self.cur_episode, self.t, self.dt, action, global_reward))
 
     def _log_traffic_data(self):
-        import pandas as pd
-        tr = np.array(self._trace)                 # [steps, 3, N]
-        hs, vs, us = tr[:, 0], tr[:, 1], tr[:, 2]
-        df = pd.DataFrame()
-        df['episode'] = np.ones(len(hs)) * self.cur_episode
-        df['time_sec'] = np.arange(len(hs)) * self.dt
-        df['reward'] = np.array(self.rewards)
-        df['lead_headway_m'] = hs[:, 0]
-        df['avg_headway_m'] = np.mean(hs[:, 1:], axis=1)
-        df['std_headway_m'] = np.std(hs[:, 1:], axis=1)
-        df['avg_speed_mps'] = np.mean(vs, axis=1)
-        df['std_speed_mps'] = np.std(vs, axis=1)
-        df['avg_accel_mps2'] = np.mean(us, axis=1)
-        df['std_accel_mps2'] = np.std(us, axis=1)
-        for i in range(self.n_agent):
-            df['headway_%d_m' % (i + 1)] = hs[:, i]
-            df['velocity_%d_mps' % (i + 1)] = vs[:, i]
-            df['accel_%d_mps2' % (i + 1)] = us[:, i]
-        self.traffic_data.append(df)
+        self.traffic_data.append(traffic_frame(self.cur_episode, self.dt, self.rewards, np.array(self._trace),
+                                               self.n_agent))
+
+    def record_episode(self, episode, actions, global_rewards, trace):
+        """Append one finished episode recorded elsewhere (the batched evaluator) to the same records the
+        step-by-step path builds.  actions [steps, N], global_rewards float64 [steps], trace float64
+        [steps + 1, 3, N] with the reset state first."""
+        for s in range(len(global_rewards)):
+            self.control_data.append(control_row(episode, s + 1, self.dt, actions[s], global_rewards[s]))
+        self.traffic_data.append(traffic_frame(episode, self.dt, [0] + list(global_rewards), trace, self.n_agent))
 
     def output_data(self):
         import pandas as pd

@@ -9,7 +9,8 @@ bootstrap at a non-terminal batch end is one more policy + value call, Q4 the re
 that of a greedy test episode run after every training episode, Q5 only training steps are counted.
 
 ``VecTrainer`` is the batched loop this package adds (n_env parallel episodes, everything device resident,
-optionally one process per GPU with one NCCL gradient all-reduce per update).
+optionally one process per GPU with one NCCL gradient all-reduce per update).  ``VecEvaluator`` runs the greedy
+test episodes of many seeds as one device batch, with the per-seed results of ``Evaluator``.
 """
 import logging
 import pathlib
@@ -18,6 +19,8 @@ import time
 
 import numpy as np
 import torch
+
+from . import _lib as L
 
 _TEST_MODES = {'no_test': (False, False), 'in_train_test': (True, False),
                'after_train_test': (False, True), 'all_test': (True, True)}
@@ -94,6 +97,18 @@ class Counter:
 
     def should_stop(self):
         return self.stop or self.cur_step >= self.total_step
+
+
+def eval_due(n_update, per_update, eval_interval, total_step):
+    """Cadence of the batched trainer's greedy evaluations (TRAIN_CONFIG.eval_interval, in environment steps):
+    True after the update that reaches or crosses a multiple of eval_interval, and after the final update
+    (the one that reaches total_step).  Never when eval_interval is absent or 0."""
+    if not eval_interval or eval_interval <= 0:
+        return False
+    done = int(n_update) * int(per_update)
+    if done >= total_step:
+        return True
+    return done // int(eval_interval) > (done - int(per_update)) // int(eval_interval)
 
 
 # ---- the single-environment loop -----------------------------------------------------------------------------------
@@ -289,6 +304,8 @@ class VecTrainer:
             raise AssertionError('VecTrainer: episode length %d / env batch_size %d are not multiples of the update '
                                  'length %d' % (env.T, env.batch_size, model.n_step))
         self.data = []                     # one record per update (train_reward.csv of the batched loop)
+        self.eval_data = []                # one record per test seed and evaluation (eval_reward.csv)
+        self.evaluator = None
 
     def start(self):
         self._seed = self.env.seed
@@ -345,6 +362,136 @@ class VecTrainer:
             summary_writer.add_scalar('train_reward', mean, int(global_step))
         return mean
 
+    def evaluate(self, global_step, summary_writer=None):
+        """One greedy episode on each of ENV_CONFIG.test_seeds with the current weights (``VecEvaluator``: own env,
+        LSTM states and buffers; the training state, RNG and buffers are not touched).  Appends one
+        `eval_reward.csv` record per seed (``test_id`` = index into test_seeds) and writes the TB scalar
+        `test_reward`, the mean over seeds, which it returns.  Host sync."""
+        if self.evaluator is None:
+            self.evaluator = VecEvaluator(self.env.config, self.model, self.env.test_seeds)
+        res = self.evaluator.run()
+        for k, (mean, std) in enumerate(res):
+            self.eval_data.append(dict(agent=self.env.agent, step=int(global_step), test_id=k, avg_reward=mean,
+                                       std_reward=std))
+        mean = float(np.mean([m for m, _ in res]))
+        if summary_writer is not None:
+            summary_writer.add_scalar('test_reward', mean, int(global_step))
+        return mean
+
     def write_csv(self, output_path):
         import pandas as pd
         pd.DataFrame(self.data).to_csv(output_path + 'train_reward.csv')
+        if self.eval_data:
+            pd.DataFrame(self.eval_data).to_csv(output_path + 'eval_reward.csv')
+
+
+def _gather_layout(layout):
+    """The layout of the same parameters with observations gathered on the device (IA2C's 'concat' API mode
+    packs the same flat parameters; the batched episode has no host-side concatenation)."""
+    if layout.obs_mode == 'gather':
+        return layout
+    from .layout import ModelLayout
+    g = ModelLayout(layout.variant, layout.n_s_ls, layout.n_a, layout.mask, obs_mode='gather')
+    assert g.entries == layout.entries and g.n_param == layout.n_param, 'gather layout moves the parameters'
+    return g
+
+
+class VecEvaluator:
+    """Greedy test episodes of B = len(seeds) seeds advancing together on the device, forward only.
+
+    Seed k gives what ``Trainer.perform`` / ``Evaluator`` give for it, bit for bit: the reset draws the same
+    uniforms (``CACCEnv.reset_seeds``), the policy runs the FFMA cell kernel whose rows do not depend on B (the
+    tensor-core path is never used here, so a seed's trajectory does not depend on how many seeds share its batch),
+    the greedy choice is np.argmax's first maximum, and mean / std are taken on the host over the episode's steps.
+
+    The engine reads the model's ``params`` tensor itself (shared, not copied), so an evaluation during training
+    sees the current weights; LSTM states, DIAL messages, the obs / fingerprint / done / action buffers, the Philox
+    counter and the env are its own.  The episode runs in chunks of ENV_CONFIG.batch_size steps (an episode can end
+    only at such a boundary or at T) with no host synchronisation inside a chunk; after a chunk one small read
+    decides whether every env is done."""
+
+    def __init__(self, env_config, model, seeds):
+        from .agents.engine import PolicyEngine
+        from .envs.cacc_env import CACCEnv
+        self.seeds = [int(s) for s in seeds]
+        if not self.seeds:
+            raise ValueError('VecEvaluator needs at least one seed')
+        src = model.engine
+        rng_state = np.random.get_state()      # CACCEnv seeds the global stream (reference behaviour): keep it as it was
+        try:
+            self.env = CACCEnv(env_config, n_env=len(self.seeds), device=src.device)
+        finally:
+            np.random.set_state(rng_state)
+        self.env.init_test_seeds(self.seeds)
+        self.T, self.chunk = self.env.T, self.env.batch_size
+        lay = _gather_layout(model.layout)
+        self.engine = PolicyEngine(lay, len(self.seeds), self.T, src.hp, flat_params=np.zeros(lay.n_param, np.float32),
+                                   device=src.device, distance_mask=self.env.distance_mask,
+                                   coop_gamma=self.env.coop_gamma, use_tc=False)
+        self.engine.params = src.params
+        self.trace = None
+
+    def begin(self, record=False):
+        """Reset every env to its seed's test episode, the recurrent state to zero, pre-step done = 1 and the
+        fingerprints to 1/n_a (reset + model.reset() of ``Trainer.perform``)."""
+        e, env = self.engine, self.env
+        env.reset_seeds(self.seeds, obs_out=e.obs_buf[0], fp_out=e.fp_buf[0])
+        e.reset_states()
+        e.done_buf[0].fill_(1.0)
+        self.trace = None
+        if record:
+            N, B = env.n_agent, env.n_env
+            self.trace = torch.zeros(self.T + 1, 3, N, B, dtype=torch.float64, device=e.device)
+            torch.stack((env.hs, env.vs, env.us), out=self.trace[0])
+
+    def run_chunk(self, t0):
+        """Steps t0 .. t0 + batch_size - 1 (at most up to T), launches only; returns the step reached."""
+        e, env = self.engine, self.env
+        t1 = min(t0 + self.chunk, self.T)
+        for t in range(t0, t1):
+            # greedy p-call; pi goes straight into the next step's fingerprint slot (env.update_fingerprint)
+            e.step_p(e.obs_buf[t], e.fp_buf[t], e.done_buf[t], e.fp_buf[t + 1], e.act_buf[t], L.SAMPLE_GREEDY)
+            env.step_device(e.act_buf[t], obs_out=e.obs_buf[t + 1], reward_out=e.rew_buf[t],
+                            greward_out=e.grew_buf[t], done_out=e.done_buf[t + 1])
+            if self.trace is not None:
+                torch.stack((env.hs, env.vs, env.us), out=self.trace[t + 1])
+        return t1
+
+    def all_done(self, t):
+        """Host sync: has every env's episode ended within steps 1..t?"""
+        return bool(self.engine.done_buf[1:t + 1].amax(dim=0).min().item())
+
+    def run(self, record=False):
+        """One greedy episode per seed -> list of per-seed (mean, std) of the per-step global reward, over the
+        steps up to and including the episode's first done.  With record=True the episodes are also appended,
+        in seed order as episodes 1..B, to the env's records (``env.init_data`` first; ``env.output_data()``
+        writes them)."""
+        self.begin(record)
+        t = 0
+        while t < self.T:
+            t = self.run_chunk(t)
+            if t < self.T and self.all_done(t):
+                break
+        e = self.engine
+        done = e.done_buf[1:t + 1].cpu().numpy()                       # [t, B]
+        grew = np.ascontiguousarray(e.grew_buf[:t].cpu().numpy().T)     # [B, t]
+        steps = done.argmax(axis=0) + 1                                 # first done (an env is done at T at the latest)
+        assert done[steps - 1, np.arange(len(self.seeds))].all(), 'an episode did not end'
+        self.steps = [int(n) for n in steps]                            # episode length per seed
+        # contiguous per-seed rows: NumPy's reductions then sum in the same order as on the sequential path's arrays
+        res = [(np.mean(grew[k, :n]), np.std(grew[k, :n])) for k, n in enumerate(steps)]
+        if record:
+            acts = np.ascontiguousarray(np.transpose(e.act_buf[:t].cpu().numpy(), (2, 0, 1)))         # [B, t, N]
+            trace = np.ascontiguousarray(np.transpose(self.trace[:t + 1].cpu().numpy(), (3, 0, 1, 2)))  # [B, t+1, 3, N]
+            for k, n in enumerate(steps):
+                self.env.record_episode(k + 1, acts[k, :n], grew[k, :n], trace[k, :n + 1])
+        return res
+
+    def evaluate(self, output_path, gui=False):
+        """``Evaluator.run`` for the whole batch: the same log lines and the same control / traffic files."""
+        self.env.init_data(not gui, False, output_path)
+        res = self.run(record=not gui)
+        for k, (reward, _) in enumerate(res):
+            logging.info('test %i, avg reward %.2f' % (k, reward))
+        self.env.output_data()
+        return res
