@@ -69,13 +69,13 @@ class BwdArgs(C.Structure):
                 ('wt', C.c_void_p), ('ws', C.c_void_p), ('ws_floats', C.c_int64),
                 ('loss_part', C.c_void_p), ('grads', C.c_void_p), ('wpack', C.c_void_p), ('tc_err', C.c_void_p),
                 ('sv_dzT', C.c_void_p), ('sv_dpT', C.c_void_p), ('state_fm', C.c_int32),
-                ('ctx', C.c_void_p), ('raw_tiles', C.c_int32), ('ev_step', C.c_void_p), ('ev_wgrad', C.c_void_p), ('fused_heads', C.c_int32)]
+                ('ctx', C.c_void_p), ('ev_step', C.c_void_p), ('ev_wgrad', C.c_void_p), ('fused_heads', C.c_int32)]
 
 
 _lib = None
 
 EXPORTS = ['nmarl_last_error', 'nmarl_version', 'nmarl_create', 'nmarl_destroy', 'nmarl_sizeof_bwd_args', 'nmarl_sizeof_fwd_args', 'nmarl_sizeof_model', 'nmarl_sizeof_agent', 'nmarl_sizeof_cacc_cfg',
-           'nmarl_cacc_reset', 'nmarl_cacc_step', 'nmarl_pack_weights', 'nmarl_policy_step_p', 'nmarl_policy_step_v', 'nmarl_dial_msg',
+           'nmarl_cacc_reset', 'nmarl_cacc_step', 'nmarl_pack_weights', 'nmarl_policy_step_p', 'nmarl_policy_step_v', 'nmarl_tc_supported', 'nmarl_dial_msg',
            'nmarl_rng_advance', 'nmarl_nstep_return_adv', 'nmarl_loss_tiles', 'nmarl_ws_floats',
            'nmarl_a2c_backward', 'nmarl_a2c_train_forward', 'nmarl_a2c_bptt', 'nmarl_a2c_train_heads',
            'nmarl_clip_rmsprop_step', 'nmarl_consensus_update']
@@ -99,6 +99,7 @@ def lib():
     L.nmarl_cacc_step.argtypes = [C.POINTER(CaccCfg), I, I, P, P, P, P, P, P, P, P, I, P, P, P, P]
     L.nmarl_policy_step_p.argtypes = [C.POINTER(Model), C.POINTER(FwdArgs), P]
     L.nmarl_policy_step_v.argtypes = [C.POINTER(Model), C.POINTER(FwdArgs), P]
+    L.nmarl_tc_supported.argtypes = [C.POINTER(Model), I]
     L.nmarl_dial_msg.argtypes = [C.POINTER(Model), I, P, P, P, P]
     L.nmarl_pack_weights.argtypes = [C.POINTER(Model), P, P, P, P]
     L.nmarl_rng_advance.argtypes = [P, U64, P]

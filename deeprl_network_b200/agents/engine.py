@@ -45,16 +45,15 @@ class PolicyEngine:
         self.grads = torch.zeros(layout.n_param, **f32)
         self.ms = torch.ones(layout.n_param, **f32)             # TF RMSProp slot starts at 1
         self.wt = torch.zeros(layout.n_wt, **f32)
-        # tcgen05 path: packed 3xTF32 operands; used by the kernels when B % 128 == 0
+        # tcgen05 path: packed 3xTF32 operands; the library runs it whenever wpack is passed and nmarl_tc_supported holds
         if use_tc is None:
             use_tc = os.environ.get('NMARL_NO_TC', '0') != '1'
-        # same conditions as nmarl_tc_fwd_supported / the bptt dispatch (csrc): whole 128-env tiles, narrow encoders
-        self.use_tc = bool(use_tc) and (self.B % 128 == 0) and layout.kx_pad <= 32 and layout.kp_pad <= 32
+        self.use_tc = bool(use_tc) and bool(L.lib().nmarl_tc_supported(C.byref(self.model), self.B))
         self.wpack = torch.zeros(layout.n_wp, **f32) if self.use_tc else None
         self.tc_err = torch.zeros(1, dtype=torch.int32, device=dev)
         # tensor-core path: LSTM state (and its gradients) feature-major [N,64,B] so that lane == env accesses are
         # coalesced; DIAL keeps env-major state (its message kernels are env-major)
-        self.state_fm = self.use_tc and self.variant != 'ma2c_dial' and os.environ.get('NMARL_NO_STATE_FM', '0') != '1'
+        self.state_fm = self.use_tc and self.variant != 'ma2c_dial'
         self._sshape = (N, NH, B) if self.state_fm else (N, B, NH)
         self.c = [torch.zeros(*self._sshape, **f32) for _ in range(2)]
         self.h = [torch.zeros(*self._sshape, **f32) for _ in range(2)]
@@ -98,8 +97,7 @@ class PolicyEngine:
         self.kernel_events = None          # bench.py: list collecting (start, end) CUDA events around each rollout p-call
         self.T_cur = T
         self.launches = 0
-        # single-copy operand tiles for the weight-gradient GEMMs (nmarl_bwd_args.raw_tiles)
-        self.raw_tiles = self.use_tc and os.environ.get('NMARL_RAW_TILES', '1') != '0'
+        self.raw_tiles = self.use_tc       # read by bench.py (profiles/traffic.json keys): operand tiles are raw fp32
         self.bwd_events = None             # bench.py: (step events [2T], wgrad events [2]) recorded inside nmarl_a2c_bptt
         self._ctx = C.c_void_p()
         L.check(L.lib().nmarl_create(C.byref(self._ctx)), 'nmarl_create')
@@ -342,10 +340,10 @@ class PolicyEngine:
         # tensor-core path: sv_dz holds per-tile gate-bias partial sums, sv_dpre is unused (operand tiles instead)
         self.sv_dz = z(T, N, B // 128, 4 * NH) if self.use_tc else z(T, N, B, 4 * NH)
         self.sv_dpre = z(4) if self.use_tc else z(T, N, B, 192)
-        # tensor-core path: dz / encoder pre-activation gradients additionally as K-major [hi | lo] operand tiles
+        # tensor-core path: dz / encoder pre-activation gradients additionally as K-major raw fp32 operand tiles
         ndp = {'ma2c_nc': 192, 'ia2c': 64}.get(self.variant, 128)
-        self.sv_dzT = z(T, N, B // 32, 2 * 256 * 32) if self.use_tc else None
-        self.sv_dpT = z(T, N, B // 32, 2 * ndp * 32) if self.use_tc else None
+        self.sv_dzT = z(T, N, B // 32, 256 * 32) if self.use_tc else None
+        self.sv_dpT = z(T, N, B // 32, ndp * 32) if self.use_tc else None
         self.sv_dmp = z(T, N, B, NH) if self.variant == 'ma2c_dial' else None
         self.dh_rec, self.dc_rec = z(2, *self._sshape), z(2, *self._sshape)
         self.dmsg = z(2, N, L.MAX_NBR, *self._sshape[1:]) if self.variant != 'ia2c' else None
@@ -372,7 +370,7 @@ class PolicyEngine:
         a.wpack, a.tc_err = L.ptr(self.wpack), L.ptr(self.tc_err)
         a.sv_dzT, a.sv_dpT = L.ptr(self.sv_dzT), L.ptr(self.sv_dpT)
         a.state_fm = int(self.state_fm)
-        a.ctx, a.raw_tiles = self._ctx, int(self.raw_tiles)
+        a.ctx = self._ctx
         if self.bwd_events is not None:
             step_ev, wg_ev = self.bwd_events
             self._ev_arrays = ((C.c_void_p * len(step_ev))(*[ev.cuda_event for ev in step_ev]),

@@ -13,21 +13,12 @@ void nmarl_set_error(const char* fmt, ...) {
 }
 
 extern "C" const char* nmarl_last_error(void) { return g_err; }
-extern "C" int nmarl_version(void) { return 100; }
+extern "C" int nmarl_version(void) { return 101; }
 extern "C" int nmarl_sizeof_model(void) { return (int)sizeof(nmarl_model); }
 extern "C" int nmarl_sizeof_agent(void) { return (int)sizeof(nmarl_agent); }
 extern "C" int nmarl_sizeof_cacc_cfg(void) { return (int)sizeof(nmarl_cacc_cfg); }
 extern "C" int nmarl_sizeof_fwd_args(void) { return (int)sizeof(nmarl_fwd_args); }
 extern "C" int nmarl_sizeof_bwd_args(void) { return (int)sizeof(nmarl_bwd_args); }
-
-bool nmarl_pdl_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("NMARL_NO_PDL");
-    on = (e != nullptr && e[0] == '1') ? 0 : 1;
-  }
-  return on != 0;
-}
 
 extern "C" int nmarl_create(nmarl_ctx** out) {
   NMARL_CHECK(out != nullptr, "nmarl_create: out is NULL");

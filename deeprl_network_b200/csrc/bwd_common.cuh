@@ -20,12 +20,15 @@ struct BwdK {
   float* dh_out; float* dc_out; float* dmsg_out;                       // consumed by step t-1
   float* sv_dz; float* sv_dpre;                                        // step t (tcgen05 path: sv_dz = [N][tiles][256] gate-bias partials)
   const float* wpack; int* tc_err;                                     // tcgen05 path (NULL -> FFMA)
-  float* dzT;                                                          // step t: [N][B/32][hi|lo][256][32] tiles or NULL
-  float* dpT;                                                          // step t: [N][B/32][hi|lo][ndp][32] tiles (encoder pre-act grads)
-  int state_fm;                                                        // c/dh/dc/dmsg tensors are feature-major
+  float* dzT;                                                          // step t: [N][B/32][256][32] raw fp32 tiles or NULL
+  float* dpT;                                                          // step t: [N][B/32][ndp][32] raw fp32 tiles (encoder pre-act grads)
   int ndp;                                                             // rows of a dpT tile: 192 (NC) / 128 (IC3, DIAL) / 64 (IA2C)
-  int raw_tiles;                                                       // experimental (NMARL_RAW_TILES): dzT/dpT hold one raw fp32 tile, no [hi|lo] pair
 };
+
+// floats per time step of sv_dzT (rows = 256) / sv_dpT (rows = ndp): one rows x 32 tile per agent and 32 envs
+__host__ __device__ inline size_t nmarl_tc_tile_step_floats(int n_agent, int B, int rows) {
+  return (size_t)n_agent * (B / 32) * rows * 32;
+}
 
 int nmarl_tc_launch_bwd(const nmarl_model* m, const BwdK& k, cudaStream_t st);
 int nmarl_tc_wgrad_splits(int n_agent);
@@ -34,5 +37,5 @@ int nmarl_tc_ndp(const nmarl_model* m);
 // all GEMM weight gradients (gate + encoders) of the tensor-core path; activations are feature-major
 int nmarl_tc_launch_wgrads(const nmarl_model* m, int B, int T, const float* sv_sh, const float* sv_xin, const float* dzT,
                            const float* dpT, const float* sv_dz, float* ws, float* grads, int* err, cudaStream_t st, cudaStream_t st_bias,
-                           bool raw_tiles = false, void** ev_wgrad = nullptr,
+                           void** ev_wgrad = nullptr,
                            const float* h_seq = nullptr, const float* done_pre = nullptr);

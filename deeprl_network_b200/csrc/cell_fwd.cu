@@ -473,7 +473,8 @@ extern "C" int nmarl_policy_step_p(const nmarl_model* m, const nmarl_fwd_args* a
   NMARL_CHECK(m->variant != NMARL_DIAL || (a->msg_in && a->msg_out), "policy_step_p: DIAL needs msg_in/msg_out");
   NMARL_CHECK(a->sample_mode != NMARL_SAMPLE_UNIFORM || a->uniforms, "policy_step_p: uniforms required");
   NMARL_CHECK(a->sample_mode != NMARL_SAMPLE_PHILOX || a->rng, "policy_step_p: rng state required");
-  NMARL_CHECK(!a->state_fm || nmarl_tc_fwd_supported(m, a), "policy_step_p: feature-major state needs the tensor-core path");
+  const int fm = nmarl_state_fm(m, nmarl_tc_fwd_supported(m, a));
+  NMARL_CHECK(a->state_fm == fm, "policy_step_p: state_fm must be %d for this variant and path, got %d", fm, a->state_fm);
   FwdK k{};
   k.a = *a;
   if (a->sv_sh != nullptr) {                 // rollout p-call that also saves activations for BPTT
@@ -492,7 +493,8 @@ extern "C" int nmarl_policy_step_v(const nmarl_model* m, const nmarl_fwd_args* a
               "policy_step_v: missing buffers");
   NMARL_CHECK((m->variant != NMARL_NC && m->variant != NMARL_DIAL) || a->fp, "policy_step_v: fp required");
   NMARL_CHECK(m->variant != NMARL_DIAL || a->msg_in, "policy_step_v: DIAL needs msg_in");
-  NMARL_CHECK(!a->state_fm || nmarl_tc_fwd_supported(m, a), "policy_step_v: feature-major state needs the tensor-core path");
+  const int fm = nmarl_state_fm(m, nmarl_tc_fwd_supported(m, a));
+  NMARL_CHECK(a->state_fm == fm, "policy_step_v: state_fm must be %d for this variant and path, got %d", fm, a->state_fm);
   FwdK k{};
   k.a = *a;
   return dispatch_fwd<MODE_V>(m, k, (cudaStream_t)stream);

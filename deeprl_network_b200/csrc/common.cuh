@@ -49,9 +49,11 @@ void nmarl_set_error(const char* fmt, ...);
     }                                                                                       \
   } while (0)
 
+// LSTM-state layout (nmarl_fwd_args / nmarl_bwd_args.state_fm) the kernels implement: feature-major on the
+// tensor-core path, except DIAL, whose message kernels are env-major; env-major on the FFMA path
+inline int nmarl_state_fm(const nmarl_model* m, bool tc) { return (tc && m->variant != NMARL_DIAL) ? 1 : 0; }
+
 // ---- kernel launch with optional programmatic dependent launch (see tc.cuh: pdl_wait) ---------------------------
-// NMARL_NO_PDL=1 in the environment turns the attribute off (A/B switch; the device-side instructions become no-ops).
-bool nmarl_pdl_enabled();
 template <typename... KArgs, typename... Args>
 inline cudaError_t nmarl_launch(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, bool pdl,
                                 Args&&... args) {
@@ -61,7 +63,7 @@ inline cudaError_t nmarl_launch(void (*kern)(KArgs...), dim3 grid, dim3 block, s
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
-  cfg.numAttrs = (pdl && nmarl_pdl_enabled()) ? 1 : 0;
+  cfg.numAttrs = pdl ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 

@@ -10,9 +10,9 @@
 namespace {
 using namespace tcrow;
 
-// RAW (experimental, DESIGN.md 6.2): the operand tiles for the weight-gradient GEMMs are stored once as raw fp32
-// instead of as a [hi | lo] pair; the weight-gradient kernel derives lo in shared memory.
-template <int VAR, bool FM, bool RAW>
+// The operand tiles for the weight-gradient GEMMs (dzT, dpT) are stored once as raw fp32; the weight-gradient kernel
+// derives the 3xTF32 lo part in shared memory (tc_wgrad.cu).
+template <int VAR, bool FM>
 __global__ void __launch_bounds__(TC_THREADS, 1) tc_cell_bwd_kernel(const __grid_constant__ nmarl_model m,
                                                                     const __grid_constant__ BwdK k) {
   extern __shared__ uint8_t smem_raw[];
@@ -146,19 +146,12 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_cell_bwd_kernel(const __grid
         const int col = (((lane >> 4) & 1) << 3) | (((lane >> 3) & 1) << 2) | (((lane >> 2) & 1) << 1) | ((lane >> 1) & 1);
         if ((lane & 1) == 0) bsum[quarter * NG + g * NH + e0 + col] = a[0];
       }
-      if (k.dzT != nullptr) {                 // dz^T tile for the tensor-core wgrad: K-major over rows, hi | lo
-        uint8_t* tile = reinterpret_cast<uint8_t*>(k.dzT) + ((size_t)i * (B / 32) + (b0 / 32) + quarter) * (size_t)((RAW ? 1 : 2) * 256 * 128);
+      if (k.dzT != nullptr) {                 // dz^T tile for the tensor-core wgrad: K-major over rows, raw fp32
+        uint8_t* tile = reinterpret_cast<uint8_t*>(k.dzT) + ((size_t)i * (B / 32) + (b0 / 32) + quarter) * (size_t)(256 * 128);
 #pragma unroll
         for (int j = 0; j < EW; ++j) {
           const uint32_t off = tc::sw128_offset((uint32_t)(g * NH + e0 + j), (uint32_t)lane);
-          if constexpr (RAW) {
-            __stcs(reinterpret_cast<float*>(tile + off), dz[j]);
-          } else {
-            float hi, lo;
-            tc::split_tf32(dz[j], hi, lo);
-            __stcs(reinterpret_cast<float*>(tile + off), hi);                       // read once, by the wgrad kernel
-            __stcs(reinterpret_cast<float*>(tile + 256 * 128 + off), lo);
-          }
+          __stcs(reinterpret_cast<float*>(tile + off), dz[j]);                      // read once, by the wgrad kernel
         }
       }
       produce_act(c, dz);                      // the gate's two k-blocks of the 256-deep dgrad contraction
@@ -201,20 +194,13 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_cell_bwd_kernel(const __grid
 #pragma unroll
     for (int j = 0; j < EW; ++j) dpm[j] = 0.f;
     uint8_t* dptile = (k.dpT != nullptr)
-        ? reinterpret_cast<uint8_t*>(k.dpT) + ((size_t)i * (B / 32) + (b0 / 32) + quarter) * (size_t)((RAW ? 1 : 2) * k.ndp * 128) : nullptr;
+        ? reinterpret_cast<uint8_t*>(k.dpT) + ((size_t)i * (B / 32) + (b0 / 32) + quarter) * (size_t)(k.ndp * 128) : nullptr;
     auto put_dp = [&](int n0, const float (&vals)[EW]) {        // encoder pre-activation grads as K-major tiles
       if (dptile == nullptr) return;
 #pragma unroll
       for (int j = 0; j < EW; ++j) {
         const uint32_t off = tc::sw128_offset((uint32_t)(n0 + j), (uint32_t)lane);
-        if constexpr (RAW) {
-          __stcs(reinterpret_cast<float*>(dptile + off), vals[j]);
-        } else {
-          float hi, lo;
-          tc::split_tf32(vals[j], hi, lo);
-          __stcs(reinterpret_cast<float*>(dptile + off), hi);
-          __stcs(reinterpret_cast<float*>(dptile + (size_t)k.ndp * 128 + off), lo);
-        }
+        __stcs(reinterpret_cast<float*>(dptile + off), vals[j]);
       }
     };
 #pragma unroll
@@ -292,9 +278,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_cell_bwd_kernel(const __grid
   if (warp == ROW_THREADS / 32 + 1) { tc::fence_after_sync(); tc::tmem_dealloc(tmem, 512); }
 }
 
-template <int VAR, bool FM, bool RAW>
-int launch_tc_bwd_fm(const nmarl_model* m, const BwdK& k, cudaStream_t st) {
-  auto kern = tc_cell_bwd_kernel<VAR, FM, RAW>;
+// one state layout per variant: feature-major except DIAL, whose message kernels are env-major
+template <int VAR>
+int launch_tc_bwd(const nmarl_model* m, const BwdK& k, cudaStream_t st) {
+  auto kern = tc_cell_bwd_kernel<VAR, VAR != NMARL_DIAL>;
   static bool configured = false;
   if (!configured) {
     NMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM));
@@ -304,12 +291,6 @@ int launch_tc_bwd_fm(const nmarl_model* m, const BwdK& k, cudaStream_t st) {
   NMARL_CUDA(nmarl_launch(kern, grid, dim3(TC_THREADS), TC_SMEM, st, true, *m, k));
   NMARL_LAUNCH_CHECK();
   return 0;
-}
-
-template <int VAR>
-int launch_tc_bwd(const nmarl_model* m, const BwdK& k, cudaStream_t st) {
-  if (k.raw_tiles) return k.state_fm ? launch_tc_bwd_fm<VAR, true, true>(m, k, st) : launch_tc_bwd_fm<VAR, false, true>(m, k, st);
-  return k.state_fm ? launch_tc_bwd_fm<VAR, true, false>(m, k, st) : launch_tc_bwd_fm<VAR, false, false>(m, k, st);
 }
 
 }  // namespace

@@ -486,9 +486,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_cell_fwd_kernel(const __grid
 }
 
 
-template <int VAR, int MODE, bool FM>
-int launch_tc_fm(const nmarl_model* m, const FwdK& k, cudaStream_t st) {
-  auto kern = tc_cell_fwd_kernel<VAR, MODE, FM>;
+// one state layout per variant: feature-major except DIAL, whose message kernels are env-major
+template <int VAR, int MODE>
+int launch_tc(const nmarl_model* m, const FwdK& k, cudaStream_t st) {
+  auto kern = tc_cell_fwd_kernel<VAR, MODE, VAR != NMARL_DIAL>;
   static bool configured = false;
   if (!configured) {
     NMARL_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM));
@@ -500,11 +501,6 @@ int launch_tc_fm(const nmarl_model* m, const FwdK& k, cudaStream_t st) {
   NMARL_CUDA(nmarl_launch(kern, grid, dim3(TC_THREADS), TC_SMEM, st, true, *m, k2));
   NMARL_LAUNCH_CHECK();
   return 0;
-}
-
-template <int VAR, int MODE>
-int launch_tc(const nmarl_model* m, const FwdK& k, cudaStream_t st) {
-  return k.a.state_fm ? launch_tc_fm<VAR, MODE, true>(m, k, st) : launch_tc_fm<VAR, MODE, false>(m, k, st);
 }
 
 template <int VAR>
@@ -519,11 +515,15 @@ int launch_tc_mode(const nmarl_model* m, const FwdK& k, int mode, cudaStream_t s
 
 }  // namespace
 
-bool nmarl_tc_fwd_supported(const nmarl_model* m, const nmarl_fwd_args* a) {
-  if (a->wpack == nullptr || a->B % 128 != 0 || m->kx_pad > 32 || m->kp_pad > 32) return false;
+extern "C" int nmarl_tc_supported(const nmarl_model* m, int B) {
+  if (B % 128 != 0 || m->kx_pad > 32 || m->kp_pad > 32) return 0;
   for (int i = 0; i < m->n_agent; ++i)
-    if (m->agent[i].tp_g < 0 || m->agent[i].tp_x < 0) return false;
-  return true;
+    if (m->agent[i].tp_g < 0 || m->agent[i].tp_x < 0) return 0;
+  return 1;
+}
+
+bool nmarl_tc_fwd_supported(const nmarl_model* m, const nmarl_fwd_args* a) {
+  return a->wpack != nullptr && nmarl_tc_supported(m, a->B);
 }
 
 int nmarl_tc_launch_fwd(const nmarl_model* m, const FwdK& k, int mode, cudaStream_t st) {

@@ -4,9 +4,9 @@
 // fixed-order reduce afterwards.
 //   A operand: the saved activations are feature-major ([t][agent][feature][env]); TMEM lane = feature ka, so
 //              a thread reads 8 consecutive envs (32 contiguous bytes), splits hi/lo and tcgen05.st's them.
-//   B operand: D^T, K-major over rows, was written by the backward cell kernel as ready-made [hi | lo]
-//              128B-swizzled tiles (dz: 256 rows, encoder pre-activation grads: 192/128/64 rows); the producer
-//              bulk-copies the needed row range of the tile per 32 env rows.
+//   B operand: D^T, K-major over rows, was written by the backward cell kernel as raw fp32 128B-swizzled tiles
+//              (dz: 256 rows, encoder pre-activation grads: 192/128/64 rows); the producer bulk-copies the needed
+//              row range of the tile per 32 env rows, and the 3xTF32 lo part is derived in shared memory.
 //   Biases:    the obs-encoder job carries an extra all-ones lane and spans every column of the dpre tile, which
 //              yields all encoder bias gradients for free; the gate bias is a coalesced column sum of dz.
 #include "bwd_common.cuh"
@@ -22,12 +22,12 @@ enum { J_GATE0 = 0, J_GATE1, J_ENC_X, J_ENC_M0, J_ENC_M1, J_COUNT };
 // the `lo` half of the raw B tiles in shared memory; the two dependent chains (global load -> split -> tcgen05.st
 // and TMA wait -> lds/sts -> proxy fence) run side by side instead of back to back in every thread.
 constexpr int A_SETS = 2, A_THREADS = 128 * A_SETS, WA = 32 / A_SETS;
-// Shared-memory rings.  RAW tiles: WG_RAW_STAGES single 32 KB raw tiles (bulk-copied, deep enough to cover the DRAM
-// latency of a 32 KB copy at one k-block per ~0.8 us) + WG_LO_BUFS derived `lo` tiles; [hi | lo] pairs: S_STAGES x 64 KB.
-constexpr int WG_RAW_STAGES = 5, WG_LO_BUFS = 2;
-constexpr uint32_t WG_RAW_BYTES = 256 * 128;
-constexpr size_t WG_SMEM_RAW = (size_t)(WG_RAW_STAGES + WG_LO_BUFS) * WG_RAW_BYTES + 1024 + 32 * 8 + 64;
-static_assert(WG_SMEM_RAW <= 232448, "wgrad RAW ring exceeds the 227 KB of dynamic shared memory");
+// Shared-memory rings: WG_STAGES raw 32 KB B tiles (bulk-copied, deep enough to cover the DRAM latency of a 32 KB copy
+// at one k-block per ~0.8 us) + WG_LO_BUFS derived `lo` tiles.
+constexpr int WG_STAGES = 5, WG_LO_BUFS = 2;
+constexpr uint32_t WG_TILE_BYTES = 256 * 128;
+constexpr size_t WG_SMEM = (size_t)(WG_STAGES + WG_LO_BUFS) * WG_TILE_BYTES + 1024 + 32 * 8 + 64;
+static_assert(WG_SMEM <= 232448, "wgrad ring exceeds the 227 KB of dynamic shared memory");
 constexpr int SEG_KB = 20;       // k-blocks (of 32 rows) accumulated in TMEM before the accumulator is drained (see flush)
 
 struct TcWgK {
@@ -69,24 +69,23 @@ __device__ __forceinline__ JobDesc job_desc(const nmarl_model& m, const TcWgK& k
   return d;
 }
 
-// RAW (experimental, DESIGN.md 6.2): the D^T tiles hold raw fp32 once.  The producer copies one tile per k-block; it
-// doubles as the hi operand (the TF32 datapath drops the 13 low mantissa bits -- tools/probe_tf32_operand.py); the
-// row threads derive lo = x - trunc(x) into the second half of the stage and signal lo_full; the issuer runs the two
-// passes that need only the raw tile first and a_hi * b_lo after that barrier.
-template <bool RAW>
+// The D^T tiles hold raw fp32 once.  The producer copies one tile per k-block; it doubles as the hi operand (the TF32
+// datapath drops the 13 low mantissa bits -- tools/probe_tf32_operand.py); the row threads derive lo = x - trunc(x)
+// into a lo buffer and signal lo_full; the issuer runs the two passes that need only the raw tile first and
+// a_hi * b_lo after that barrier.
 __global__ void __launch_bounds__(TC_THREADS, 1) tc_wgrad_kernel(const __grid_constant__ nmarl_model m,
                                                                  const __grid_constant__ TcWgK k) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* bst = smem;
-  constexpr int NST = RAW ? WG_RAW_STAGES : S_STAGES;                  // B stages
-  constexpr uint32_t STB = RAW ? WG_RAW_BYTES : STAGE_BYTES;           // bytes per B stage
-  uint8_t* lobuf = smem + (size_t)NST * STB;                           // RAW only: WG_LO_BUFS derived lo tiles
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (size_t)NST * STB + (RAW ? WG_LO_BUFS * WG_RAW_BYTES : 0));
+  constexpr int NST = WG_STAGES;                                       // B stages
+  constexpr uint32_t STB = WG_TILE_BYTES;                              // bytes per B stage
+  uint8_t* lobuf = smem + (size_t)NST * STB;                           // WG_LO_BUFS derived lo tiles
+  uint64_t* bars = reinterpret_cast<uint64_t*>(lobuf + (size_t)WG_LO_BUFS * STB);
   uint64_t* b_full = bars, *b_empty = bars + NST, *a_full = bars + 2 * NST, *a_empty = a_full + A_SLOTS;
   uint64_t* enc_full = a_empty + A_SLOTS, *acc_full = enc_full + 1;
   uint64_t* acc_free = acc_full + 1;                                   // accumulator drained by the row threads (segment flush)
-  uint64_t* lo_full = acc_free + 1, *lo_empty = lo_full + WG_LO_BUFS;  // RAW only
+  uint64_t* lo_full = acc_free + 1, *lo_empty = lo_full + WG_LO_BUFS;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(lo_empty + WG_LO_BUFS);
 
   const int sp = blockIdx.x, jslot = blockIdx.y, i = blockIdx.z;
@@ -107,8 +106,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_wgrad_kernel(const __grid_co
     tc::mbar_init(enc_full, 1);
     tc::mbar_init(acc_full, 1);
     tc::mbar_init(acc_free, ROW_THREADS);
-    if constexpr (RAW)
-      for (int s = 0; s < WG_LO_BUFS; ++s) { tc::mbar_init(&lo_full[s], ROW_THREADS - A_THREADS); tc::mbar_init(&lo_empty[s], 1); }
+    for (int s = 0; s < WG_LO_BUFS; ++s) { tc::mbar_init(&lo_full[s], ROW_THREADS - A_THREADS); tc::mbar_init(&lo_empty[s], 1); }
     tc::fence_barrier_init();
   }
   if (warp == ROW_THREADS / 32 + 1) tc::tmem_alloc(tmem_slot, 512);
@@ -116,14 +114,11 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_wgrad_kernel(const __grid_co
   __syncthreads();
   tc::fence_after_sync();
   const uint32_t tmem = *tmem_slot;
-  const uint32_t tile_bytes = (uint32_t)d.N * 128u;                   // hi (or lo) part staged per k-block
-  // byte offset of the D^T tile of (t, 32-env block rb): [hi | lo] pairs, or single raw tiles packed inside each
-  // time step's (unchanged) [hi | lo]-sized slab
+  const uint32_t tile_bytes = (uint32_t)d.N * 128u;                   // rows of the tile staged per k-block
+  // the D^T tile of (t, 32-env block rb)
   auto bt_tile = [&](int t, int rb) -> const uint8_t* {
-    const size_t pair = (size_t)(2 * d.tile_rows * 128);
-    const size_t off = RAW ? (size_t)t * N_agents * bpt * pair + ((size_t)i * bpt + rb) * (pair / 2)
-                           : (((size_t)t * N_agents + i) * bpt + rb) * pair;
-    return reinterpret_cast<const uint8_t*>(d.BT) + off;
+    const float* tile = d.BT + t * nmarl_tc_tile_step_floats(N_agents, k.B, d.tile_rows) + ((size_t)i * bpt + rb) * d.tile_rows * 32;
+    return reinterpret_cast<const uint8_t*>(tile);
   };
 
   if (warp < ROW_THREADS / 32) {
@@ -240,25 +235,23 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_wgrad_kernel(const __grid_co
         if (q + 1 < nkb) emit_a(q + 1, xb);
       }
     } else {
-      // ---- lo derivation (RAW tiles): lo = rn_tf32(x - trunc_tf32(x)) of the k-block's B stage ---------------------------
+      // ---- lo derivation: lo = rn_tf32(x - trunc_tf32(x)) of the k-block's B stage -----------------------------------
       const int lt = tid - A_THREADS;
       for (int q = 0; q < nkb; ++q) {
-        if constexpr (RAW) {
-          const int st = q % NST, lb = q % WG_LO_BUFS;
-          tc::mbar_wait(&lo_empty[lb], ((q / WG_LO_BUFS) & 1) ^ 1, k.err, 42);      // the MMAs that read this lo buffer are done
-          tc::mbar_wait(&b_full[st], (q / NST) & 1, k.err, 41);
-          const float4* raw = reinterpret_cast<const float4*>(bst + (size_t)st * STB);
-          float4* lo = reinterpret_cast<float4*>(lobuf + (size_t)lb * WG_RAW_BYTES);
-          for (uint32_t e = (uint32_t)lt; e < tile_bytes / 16; e += ROW_THREADS - A_THREADS) {
-            const float4 v = raw[e];
-            float4 l;
-            l.x = tc::tf32_lo_of_raw(v.x); l.y = tc::tf32_lo_of_raw(v.y);
-            l.z = tc::tf32_lo_of_raw(v.z); l.w = tc::tf32_lo_of_raw(v.w);
-            lo[e] = l;
-          }
-          tc::fence_proxy_async();
-          tc::mbar_arrive(&lo_full[lb]);
+        const int st = q % NST, lb = q % WG_LO_BUFS;
+        tc::mbar_wait(&lo_empty[lb], ((q / WG_LO_BUFS) & 1) ^ 1, k.err, 42);      // the MMAs that read this lo buffer are done
+        tc::mbar_wait(&b_full[st], (q / NST) & 1, k.err, 41);
+        const float4* raw = reinterpret_cast<const float4*>(bst + (size_t)st * STB);
+        float4* lo = reinterpret_cast<float4*>(lobuf + (size_t)lb * STB);
+        for (uint32_t e = (uint32_t)lt; e < tile_bytes / 16; e += ROW_THREADS - A_THREADS) {
+          const float4 v = raw[e];
+          float4 l;
+          l.x = tc::tf32_lo_of_raw(v.x); l.y = tc::tf32_lo_of_raw(v.y);
+          l.z = tc::tf32_lo_of_raw(v.z); l.w = tc::tf32_lo_of_raw(v.w);
+          lo[e] = l;
         }
+        tc::fence_proxy_async();
+        tc::mbar_arrive(&lo_full[lb]);
         if ((q + 1) % SEG_KB == 0 || q + 1 == nkb) flush(q / SEG_KB);
       }
     }
@@ -273,14 +266,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_wgrad_kernel(const __grid_co
         const int t = kb / bpt, rb = kb - t * bpt;
         tc::mbar_wait(&b_empty[st], ((q / NST) & 1) ^ 1, k.err, 21);
         const uint8_t* tile = bt_tile(t, rb);
-        if constexpr (RAW) {
-          tc::mbar_arrive_expect_tx(&b_full[st], tile_bytes);
-          tc::bulk_g2s(bst + (size_t)st * STB, tile + (size_t)d.n_row0 * 128, tile_bytes, &b_full[st]);
-        } else {
-          tc::mbar_arrive_expect_tx(&b_full[st], 2 * tile_bytes);
-          tc::bulk_g2s(bst + (size_t)st * STB, tile + (size_t)d.n_row0 * 128, tile_bytes, &b_full[st]);
-          tc::bulk_g2s(bst + (size_t)st * STB + tile_bytes, tile + (size_t)(d.tile_rows + d.n_row0) * 128, tile_bytes, &b_full[st]);
-        }
+        tc::mbar_arrive_expect_tx(&b_full[st], tile_bytes);
+        tc::bulk_g2s(bst + (size_t)st * STB, tile + (size_t)d.n_row0 * 128, tile_bytes, &b_full[st]);
       }
     }
   } else {
@@ -297,33 +284,23 @@ __global__ void __launch_bounds__(TC_THREADS, 1) tc_wgrad_kernel(const __grid_co
         tc::mbar_wait(&a_full[slot], (q / A_SLOTS) & 1, k.err, 32);
         tc::fence_after_sync();
         const uint64_t d_hi = tc::smem_desc_sw128(bst + (size_t)st * STB);
-        const uint64_t d_lo = tc::smem_desc_sw128(RAW ? lobuf + (size_t)lb * WG_RAW_BYTES : bst + (size_t)st * STB + tile_bytes);
-        if constexpr (RAW) {
+        const uint64_t d_lo = tc::smem_desc_sw128(lobuf + (size_t)lb * STB);
 #pragma unroll
-          for (int ks = 0; ks < 4; ++ks) {                              // passes that need only the raw tile
-            const uint32_t a_hi = tmem + A_COL + slot * 64 + ks * 8, a_lo = a_hi + 32;
-            tc::mma_tf32_ts(tmem + ACC_COL, a_hi, d_hi + 2 * ks, idesc, (seg_first && ks == 0) ? 0u : 1u);
-            tc::mma_tf32_ts(tmem + ACC_COL, a_lo, d_hi + 2 * ks, idesc, 1u);
-          }
-          if (iprof && q < 40) iprof[3 * q + 1] = clock64();
-          tc::mbar_wait(&lo_full[lb], (q / WG_LO_BUFS) & 1, k.err, 33);
-          tc::fence_after_sync();
-          if (iprof && q < 40) iprof[3 * q + 2] = clock64();
-#pragma unroll
-          for (int ks = 0; ks < 4; ++ks)
-            tc::mma_tf32_ts(tmem + ACC_COL, tmem + A_COL + slot * 64 + ks * 8, d_lo + 2 * ks, idesc, 1u);
-        } else {
-#pragma unroll
-          for (int ks = 0; ks < 4; ++ks) {
-            const uint32_t a_hi = tmem + A_COL + slot * 64 + ks * 8, a_lo = a_hi + 32;
-            tc::mma_tf32_ts(tmem + ACC_COL, a_hi, d_hi + 2 * ks, idesc, (seg_first && ks == 0) ? 0u : 1u);
-            tc::mma_tf32_ts(tmem + ACC_COL, a_hi, d_lo + 2 * ks, idesc, 1u);
-            tc::mma_tf32_ts(tmem + ACC_COL, a_lo, d_hi + 2 * ks, idesc, 1u);
-          }
+        for (int ks = 0; ks < 4; ++ks) {                                // passes that need only the raw tile
+          const uint32_t a_hi = tmem + A_COL + slot * 64 + ks * 8, a_lo = a_hi + 32;
+          tc::mma_tf32_ts(tmem + ACC_COL, a_hi, d_hi + 2 * ks, idesc, (seg_first && ks == 0) ? 0u : 1u);
+          tc::mma_tf32_ts(tmem + ACC_COL, a_lo, d_hi + 2 * ks, idesc, 1u);
         }
+        if (iprof && q < 40) iprof[3 * q + 1] = clock64();
+        tc::mbar_wait(&lo_full[lb], (q / WG_LO_BUFS) & 1, k.err, 33);
+        tc::fence_after_sync();
+        if (iprof && q < 40) iprof[3 * q + 2] = clock64();
+#pragma unroll
+        for (int ks = 0; ks < 4; ++ks)
+          tc::mma_tf32_ts(tmem + ACC_COL, tmem + A_COL + slot * 64 + ks * 8, d_lo + 2 * ks, idesc, 1u);
         tc::mma_commit(&a_empty[slot]);
         tc::mma_commit(&b_empty[st]);
-        if constexpr (RAW) tc::mma_commit(&lo_empty[lb]);
+        tc::mma_commit(&lo_empty[lb]);
         if ((q + 1) % SEG_KB == 0 || q + 1 == nkb) tc::mma_commit(acc_full);
       }
     }
@@ -415,7 +392,7 @@ int64_t nmarl_tc_wgrad_ws_floats(const nmarl_model* m) {
 
 int nmarl_tc_launch_wgrads(const nmarl_model* m, int B, int T, const float* sv_sh, const float* sv_xin, const float* dzT,
                            const float* dpT, const float* sv_dz, float* ws, float* grads, int* err, cudaStream_t st,
-                           cudaStream_t st_bias, bool raw_tiles, void** ev_wgrad, const float* h_seq, const float* done_pre) {
+                           cudaStream_t st_bias, void** ev_wgrad, const float* h_seq, const float* done_pre) {
   TcWgK k{};
   k.B = B; k.T = T; k.splits = nmarl_tc_wgrad_splits(m->n_agent); k.ndp = nmarl_tc_ndp(m);
   k.sv_sh = sv_sh; k.sv_xin = sv_xin; k.dzT = dzT; k.dpT = dpT; k.ws = ws; k.err = err;
@@ -426,15 +403,13 @@ int nmarl_tc_launch_wgrads(const nmarl_model* m, int B, int T, const float* sv_s
   for (int j = 0; j < k.n_jobs; ++j) { k.ws_off[j] = off; off += (long long)k.splits * m->n_agent * 128 * job_N(m, k.jobs[j]); }
   static bool configured = false;
   if (!configured) {
-    NMARL_CUDA(cudaFuncSetAttribute(tc_wgrad_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM));
-    NMARL_CUDA(cudaFuncSetAttribute(tc_wgrad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WG_SMEM_RAW));
+    NMARL_CUDA(cudaFuncSetAttribute(tc_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)WG_SMEM));
     configured = true;
   }
   gate_bias_reduce_kernel<<<dim3(NG / 32, m->n_agent), 256, 0, st_bias>>>(*m, sv_dz, B / 128, T, grads);   // independent of the GEMM jobs
   NMARL_LAUNCH_CHECK();
   if (ev_wgrad) NMARL_CUDA(cudaEventRecord((cudaEvent_t)ev_wgrad[0], st));
-  if (raw_tiles) tc_wgrad_kernel<true><<<dim3(k.splits, k.n_jobs, m->n_agent), TC_THREADS, WG_SMEM_RAW, st>>>(*m, k);
-  else tc_wgrad_kernel<false><<<dim3(k.splits, k.n_jobs, m->n_agent), TC_THREADS, TC_SMEM, st>>>(*m, k);
+  tc_wgrad_kernel<<<dim3(k.splits, k.n_jobs, m->n_agent), TC_THREADS, WG_SMEM, st>>>(*m, k);
   NMARL_LAUNCH_CHECK();
   if (ev_wgrad) NMARL_CUDA(cudaEventRecord((cudaEvent_t)ev_wgrad[1], st));
   NMARL_DBG_SYNC(st, "tc_wgrad_kernel");

@@ -811,8 +811,8 @@ int check_bwd_args(const nmarl_model* m, const nmarl_bwd_args* a) {
   NMARL_CHECK(m->variant == NMARL_IA2C || a->dmsg, "a2c_backward: dmsg buffer required");
   NMARL_CHECK((m->variant != NMARL_IC3 && m->variant != NMARL_DIAL) || a->sv_enc, "a2c_backward: sv_enc required");
   NMARL_CHECK(m->variant != NMARL_DIAL || (a->msg_seq && a->sv_dmp), "a2c_backward: DIAL buffers required");
-  NMARL_CHECK(!a->state_fm || (m->variant != NMARL_DIAL && a->wpack != nullptr && a->B % 128 == 0),
-              "a2c_backward: feature-major state needs the tensor-core path (and is not implemented for DIAL)");
+  const int fm = nmarl_state_fm(m, a->wpack != nullptr && nmarl_tc_supported(m, a->B));
+  NMARL_CHECK(a->state_fm == fm, "a2c_backward: state_fm must be %d for this variant and path, got %d", fm, a->state_fm);
   NMARL_CHECK((m->variant != NMARL_NC && m->variant != NMARL_DIAL) || a->fp, "a2c_backward: fp required");
   return 0;
 }
@@ -904,10 +904,11 @@ extern "C" int nmarl_a2c_bptt(const nmarl_model* m, const nmarl_bwd_args* a, voi
   const size_t nb = (size_t)N * B;
   // 0. gradients of padding slots stay zero
   NMARL_CUDA(cudaMemsetAsync(a->grads, 0, (size_t)m->n_param * sizeof(float), st));
+  // tensor-core path (reverse steps and weight gradients) or FFMA path, as in the forward (nmarl_tc_fwd_supported)
+  const bool tc = a->wpack != nullptr && nmarl_tc_supported(m, B);
   // 1. transposed weights for the FFMA backward kernels and DIAL's message-gradient kernel (the tensor-core cell
   //    kernels read their own packed transposed operands, refreshed by nmarl_pack_weights)
-  const bool tc_path = (a->wpack != nullptr && B % 128 == 0 && m->kx_pad <= 32 && m->kp_pad <= 32);
-  if (!tc_path || m->variant == NMARL_DIAL)
+  if (!tc || m->variant == NMARL_DIAL)
   for (int i = 0; i < N; ++i) {
     const nmarl_agent& ag = m->agent[i];
     dim3 blk(32, 8);
@@ -955,7 +956,6 @@ extern "C" int nmarl_a2c_bptt(const nmarl_model* m, const nmarl_bwd_args* a, voi
   }
   NMARL_CUDA(cudaEventRecord(ev_join, side));
   // 2. reverse time
-  const int raw_tiles = a->raw_tiles ? 1 : 0;      // single-copy operand tiles (DESIGN.md)
   for (int t = T - 1; t >= 0; --t) {
     BwdK k{};
     k.B = B; k.t = t; k.has_next = (t < T - 1);
@@ -975,18 +975,16 @@ extern "C" int nmarl_a2c_bptt(const nmarl_model* m, const nmarl_bwd_args* a, voi
       k.dmsg_out = a->dmsg + (size_t)pout * nb * NMARL_MAX_NBR * NH;
     }
     k.sv_dpre = a->sv_dpre + (size_t)t * nb * 192;
-    k.wpack = a->wpack; k.tc_err = a->tc_err; k.state_fm = a->state_fm;
-    k.raw_tiles = raw_tiles;
-    const bool use_tc = (a->wpack != nullptr && B % 128 == 0 && m->kx_pad <= 32 && m->kp_pad <= 32);
+    k.wpack = a->wpack; k.tc_err = a->tc_err;
     // tensor-core path: sv_dz holds the per-tile gate-bias partial sums [T][N][B/128][256]; FFMA path: dz [T][N][B][256]
-    k.sv_dz = use_tc ? a->sv_dz + (size_t)t * N * (B / 128) * NG : a->sv_dz + (size_t)t * nb * NG;
-    k.dzT = (use_tc && a->sv_dzT) ? a->sv_dzT + (size_t)t * N * (B / 32) * (2 * 256 * 32) : nullptr;
+    k.sv_dz = tc ? a->sv_dz + (size_t)t * N * (B / 128) * NG : a->sv_dz + (size_t)t * nb * NG;
     k.ndp = nmarl_tc_ndp(m);
-    k.dpT = (use_tc && a->sv_dpT) ? a->sv_dpT + (size_t)t * N * (B / 32) * (2 * k.ndp * 32) : nullptr;
+    k.dzT = (tc && a->sv_dzT) ? a->sv_dzT + t * nmarl_tc_tile_step_floats(N, B, 256) : nullptr;
+    k.dpT = (tc && a->sv_dpT) ? a->sv_dpT + t * nmarl_tc_tile_step_floats(N, B, k.ndp) : nullptr;
     int rc = 0;
     if (a->fused_heads && t == T - 1 - lead) NMARL_CUDA(cudaStreamWaitEvent(st, a->ctx->heads, 0));   // dlv of steps < T - lead
     if (a->ev_step) NMARL_CUDA(cudaEventRecord((cudaEvent_t)a->ev_step[2 * t], st));
-    if (use_tc) rc = nmarl_tc_launch_bwd(m, k, st);
+    if (tc) rc = nmarl_tc_launch_bwd(m, k, st);
     else
     switch (m->variant) {
       case NMARL_IA2C: rc = launch_bwd<NMARL_IA2C>(m, k, st); break;
@@ -1008,14 +1006,13 @@ extern "C" int nmarl_a2c_bptt(const nmarl_model* m, const nmarl_bwd_args* a, voi
   NMARL_CUDA(cudaStreamWaitEvent(st, ev_join, 0));
   int Ka[NMARL_MAX_AGENT], ow[NMARL_MAX_AGENT], ob[NMARL_MAX_AGENT];
   const int LDI = m->kx_pad + m->kp_pad + m->km_pad;
-  const bool tc_wg = (a->wpack != nullptr && B % 128 == 0 && m->kx_pad <= 32 && m->kp_pad <= 32);
-  if (tc_wg) {
+  if (tc) {
     NMARL_CHECK(a->sv_dzT && a->sv_dpT, "a2c_bptt: tensor-core path needs sv_dzT / sv_dpT");
     NMARL_CHECK(nmarl_tc_wgrad_ws_floats(m) <= a->ws_floats, "tc wgrad: workspace too small");
     // the gate-bias column sums only read sv_dz: second fork, beside the GEMM jobs
     NMARL_CUDA(cudaEventRecord(ev_fork, st));
     NMARL_CUDA(cudaStreamWaitEvent(side, ev_fork, 0));
-    if (nmarl_tc_launch_wgrads(m, B, T, a->sv_sh, a->sv_xin, a->sv_dzT, a->sv_dpT, a->sv_dz, a->ws, a->grads, a->tc_err, st, side, raw_tiles != 0, a->ev_wgrad,
+    if (nmarl_tc_launch_wgrads(m, B, T, a->sv_sh, a->sv_xin, a->sv_dzT, a->sv_dpT, a->sv_dz, a->ws, a->grads, a->tc_err, st, side, a->ev_wgrad,
                                a->state_fm ? a->h_seq : nullptr, a->done_pre)) return 1;
     NMARL_CUDA(cudaEventRecord(ev_join, side));
     NMARL_CUDA(cudaStreamWaitEvent(st, ev_join, 0));

@@ -144,16 +144,22 @@ typedef struct {
   const int32_t* act_in;   /* v-call / train: [N][B] same-step actions                         */
   float* v;                /* v-call: [N][B]                                                   */
   const float* wpack;      /* packed 3xTF32 operands (nmarl_pack_weights) or NULL.  When set and  */
-                           /* B % 128 == 0 the tcgen05 tensor-core kernel is used, else FP32 FFMA */
+                           /* nmarl_tc_supported(m, B) the tcgen05 tensor-core kernel is used,    */
+                           /* else FP32 FFMA                                                      */
   int32_t* tc_err;         /* device int: tensor-core pipeline watchdog (0 = ok); may be NULL      */
   /* optional (p-call, tensor-core path only): save the activations BPTT needs while rolling out, so the
    * update can skip the separate training forward (same inputs, same weights => same numbers):         */
   float* sv_xin; float* sv_sh; float* sv_gates; float* sv_enc;   /* step-t slices, see nmarl_bwd_args      */
-  int32_t state_fm;        /* tensor-core path only: c/h/msg tensors are feature-major [N][64][B]   */
+  int32_t state_fm;        /* 1: c/h tensors are feature-major [N][64][B].  Must be 1 on the        */
+                           /* tensor-core path except for DIAL, 0 otherwise (the call fails)      */
 } nmarl_fwd_args;
 
 int nmarl_policy_step_p(const nmarl_model* m, const nmarl_fwd_args* a, void* stream);
 int nmarl_policy_step_v(const nmarl_model* m, const nmarl_fwd_args* a, void* stream);
+/* 1 if the tensor-core kernels cover model m at B envs (whole 128-env tiles, obs / fingerprint segments of at
+ * most 32 floats, packed operands laid out for every agent), else 0.  Every entry point given a wpack runs the
+ * tensor-core path exactly when this holds; the caller sizes its buffers and state_fm by it.                */
+int nmarl_tc_supported(const nmarl_model* m, int B);
 /* Pack the GEMM weights for the tcgen05 path: per 32-wide k-block a [hi | lo] pair of 128B-swizzled
  * K-major tiles of W^T (hi = value rounded to TF32, lo = rounded remainder).  Call after every parameter
  * change.  wt (transposed weights scratch, n_wt floats) is also refreshed.                           */
@@ -210,19 +216,17 @@ typedef struct {
   float* grads;
   const float* wpack;        /* packed tensor-core operands or NULL (see nmarl_fwd_args)            */
   int32_t* tc_err;
-  float* sv_dzT;             /* tensor-core path: dz^T as [T][N][B/32][hi|lo][256][32] swizzled tiles  */
-  float* sv_dpT;             /* tensor-core path: encoder pre-activation grads^T, [T][N][B/32][hi|lo][ndp][32],
+  float* sv_dzT;             /* tensor-core path: dz^T as [T][N][B/32][256][32] swizzled raw fp32 tiles (the
+                                weight-gradient kernel derives the 3xTF32 `lo` part in shared memory)               */
+  float* sv_dpT;             /* tensor-core path: encoder pre-activation grads^T, [T][N][B/32][ndp][32] likewise,
                                 ndp = 192 (NC) / 128 (IC3, DIAL) / 64 (IA2C).  On the tensor-core path (wpack set,
-                                B % 128 == 0) sv_xin / sv_sh / sv_gates / sv_enc are FEATURE-MAJOR
+                                nmarl_tc_supported) sv_xin / sv_sh / sv_gates / sv_enc are FEATURE-MAJOR
                                 [T][N][feature][B] and sv_dpre is unused.  With state_fm the done-masked own state
                                 (rows s_dim.. of sv_sh) and, for NeurComm, the neighbour messages (the m~ block of
                                 sv_xin) are NOT stored a second time: the weight-gradient kernel reads h_seq.        */
-  int32_t state_fm;          /* tensor-core path only: h_seq / c_seq / msg_seq / dh_rec / dc_rec / dmsg are
-                                feature-major ([..][64][B] instead of [..][B][64])                                  */
+  int32_t state_fm;          /* 1: h_seq / c_seq / dh_rec / dc_rec / dmsg are feature-major ([..][64][B] instead of
+                                [..][B][64]).  Must be 1 on the tensor-core path except for DIAL, 0 otherwise        */
   nmarl_ctx* ctx;            /* required by nmarl_a2c_bptt / nmarl_a2c_backward (forked side work)                  */
-  int32_t raw_tiles;         /* tensor-core path: sv_dzT / sv_dpT hold ONE raw fp32 tile per 32 rows (the weight-
-                                gradient kernel derives the 3xTF32 `lo` part in shared memory) instead of a
-                                [hi | lo] pair: half the operand-tile traffic                                       */
   void** ev_step;            /* optional timing hooks (bench.py): 2*T cudaEvent_t, recorded on `stream` before /
                                 after the cell kernel of reverse step t at [2t], [2t+1]; NULL = none               */
   void** ev_wgrad;           /* optional: 2 cudaEvent_t around the weight-gradient GEMM kernel; NULL = none         */

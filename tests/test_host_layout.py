@@ -119,6 +119,15 @@ def test_library_loads_and_exports_header_symbols():
     assert lib.nmarl_loss_tiles(ctypes.byref(m), 4096) == 64
 
 
+def test_tc_supported_needs_whole_128_env_tiles():
+    """nmarl_tc_supported is the one rule for the tensor-core path; PolicyEngine.use_tc and the buffers it sizes follow it."""
+    lib = L.lib()
+    lay, _, _ = _layout('ma2c_nc')
+    m = lay.c_model()
+    assert lib.nmarl_tc_supported(ctypes.byref(m), 4096) == 1
+    assert lib.nmarl_tc_supported(ctypes.byref(m), 100) == 0
+
+
 def test_no_product_import_of_oracle():
     """The product package must never import the oracle (it is test infrastructure)."""
     for dirpath, _, files in os.walk(os.path.join(ROOT, 'deeprl_network_b200')):
